@@ -19,6 +19,7 @@ from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
@@ -241,6 +242,7 @@ PIXART_SIGMA = dict(num_attention_heads=16, attention_head_dim=72, in_channels=4
                     sample_size=128, caption_channels=4096)
 PIXART_BUCKETS = [(64, 64), (96, 128), (128, 128), (112, 144), (160, 160), (192, 192), (128, 96), (144, 112)]   # latent (h, w): 512^2 .. 1536^2 px
 PIXART_S_TXT = 300
+PIXART_GRAD_ACCUM = 4   # BASELINE configs[4]: a "step" of the PixArt line is one optimizer step = 4 micro-batches
 
 
 def pixart_tf_per_sample(hw, s_txt=PIXART_S_TXT):
@@ -349,7 +351,11 @@ def run_vae(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    dev_step = lambda i: vae.encode_scaled(px_dev[i % 2])
+    last = {}
+
+    def dev_step(i):
+        last["latents"] = vae.encode_scaled(px_dev[i % 2])
+
     e2e_step = lambda i: out_host.copy_(vae.encode_scaled(px_host[i % 2].to(device, non_blocking=True)))
     for i in range(args.warmup):
         dev_step(i)
@@ -360,6 +366,8 @@ def run_vae(args):
     ms = region(dev_step, args.steps)
     launches = ops.launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     e2e_step(0)
     ms_e2e = region(e2e_step, args.steps)
     if rank == 0:
@@ -442,8 +450,10 @@ def run_text(args):
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
+    last = {}
+
     def dev_step(i):
-        return encode_token_ids(clip, t5, *dev[i % 2])
+        last["prompt_embeds"], last["pooled_prompt_embeds"], _, _ = encode_token_ids(clip, t5, *dev[i % 2])
 
     def e2e_step(i):
         ci, ti = host[i % 2]
@@ -460,6 +470,8 @@ def run_text(args):
     ms = region(dev_step, args.steps)
     launches = ops.launch_count()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     e2e_step(0)
     ms_e2e = region(e2e_step, args.steps)
     if rank == 0:
@@ -492,6 +504,43 @@ def run_text(args):
 
 def batch_bytes(b):
     return int(sum(v.numel() * v.element_size() for v in b.values()))
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_MAX_ELEMS = 1 << 22   # 16 MB of float32 per output; no arm writes more than three outputs
+
+
+def flat_sample(tensors, n=DUMP_MAX_ELEMS, seed=0):
+    """The tensors flattened and concatenated in order, as float32 on the host.  When that is more than `n` elements, a
+    fixed seeded sample of `n` of them (the same positions on every run), gathered tensor by tensor so that the whole
+    concatenation (5 GB for the SD3.5 full fine-tune) is never materialised."""
+    sizes = [t.numel() for t in tensors]
+    total = sum(sizes)
+    if total <= n:
+        return torch.cat([t.detach().reshape(-1).float().cpu() for t in tensors])
+    idx = torch.randint(0, total, (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    parts, start = [], 0
+    for t, size in zip(tensors, sizes):
+        lo, hi = torch.searchsorted(idx, torch.tensor([start, start + size])).tolist()
+        if hi > lo:
+            parts.append(t.detach().reshape(-1)[(idx[lo:hi] - start).to(t.device)].float().cpu())
+        start += size
+    return torch.cat(parts)
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output as `<out_dir>/<name>.npy` in float32: a tensor that fits DUMP_MAX_ELEMS keeps its shape, a larger
+    tensor or a list of tensors (e.g. the trainable parameters) is stored as `flat_sample` of it."""
+    import numpy as np
+
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, x in outputs.items():
+        if torch.is_tensor(x) and x.numel() <= DUMP_MAX_ELEMS:
+            arr = x.detach().float().cpu()
+        else:
+            arr = flat_sample(list(x) if not torch.is_tensor(x) else [x], n=DUMP_MAX_ELEMS)
+        np.save(d / f"{name}.npy", arr.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ per-kernel timing pass
@@ -791,7 +840,7 @@ def run_b200(args):
         from simpletuner_b200.training.dist import FlatGradSync
         # full fine-tune (5 GB of gradients): 8 chunks, the optimizer of chunk i overlaps the all-reduce of chunk i + 1
         grad_sync = FlatGradSync(params, pipeline_chunks=(int(os.environ.get("STB_GRAD_CHUNKS", "8")) if sd3 else 0))
-    accum = 4 if pix else 1      # BASELINE configs[4]: grad-accum = 4 (a "step" of the PixArt line is one optimizer step = 4 micro-batches)
+    accum = PIXART_GRAD_ACCUM if pix else 1
     step = TrainStep(wrapper, opt, max_grad_norm=(0.01 if pix else 2.0), grad_clip_method="value", grad_sync=grad_sync,
                      gradient_accumulation_steps=accum)
     # auto: the two configs whose step is made of many short kernels (SD3.5-medium at 512^2, PixArt-Sigma) replay CUDA graphs
@@ -840,12 +889,6 @@ def run_b200(args):
     nbat = len(dev_batches)
     if use_graph:      # every bucket shape must be captured BEFORE the timed region
         args.warmup = max(args.warmup, nbat)
-    if (sd3 or pix) and not args.tiny:
-        # every rank must time the SAME multiset of buckets (ranks only start at different offsets): round the step count up so
-        # that the timed micro-batches are whole cycles of the bucket list
-        import math
-        cyc = nbat // math.gcd(nbat, accum)
-        args.steps = ((args.steps + cyc - 1) // cyc) * cyc
 
     def barrier():
         if world > 1:
@@ -869,10 +912,10 @@ def run_b200(args):
         return float(ms.item())
 
     per_rank_ms = []
+    last = {}
     # ---- device-resident arm
     def dev_step(i):
-        for a_ in range(accum):
-            step({k: v for k, v in dev_batches[(i * accum + a_) % nbat].items()})
+        last["loss"] = [step({k: v for k, v in dev_batches[(i * accum + a_) % nbat].items()}) for a_ in range(accum)]
 
     for i in range(args.warmup):
         dev_step(i)
@@ -893,6 +936,10 @@ def run_b200(args):
     launches = ops.launch_count()
     clocks = sampler.stop() if rank == 0 else None
     step.check_finite()
+    if args.dump_outputs and rank == 0:
+        # what a caller of the train step ends up with: the loss of each micro-batch of the last step and the trainable
+        # parameters that step's optimizer update left behind
+        dump_outputs(args.dump_outputs, {"loss": torch.stack(last["loss"]), "trainable_params": params})
 
     # ---- end-to-end arm: pinned host batch -> H2D -> step -> D2H loss, every step
     loss_host = torch.empty((), dtype=torch.float32).pin_memory()
@@ -1052,7 +1099,24 @@ def main():
     ap.add_argument("--lora-dropout", type=float, default=0.0, help="PEFT lora_dropout (flux_lora only; headline = 0.0)")
     ap.add_argument("--gradient-checkpointing", action="store_true",
                     help="re-run every block in backward like the reference's --gradient_checkpointing (not the headline config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed device-resident steps, write what the last of them computed as DIR/<name>.npy "
+                         "(float32; outputs above 4 Mi elements as a fixed seeded sample) to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200")
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.impl == "b200" and args.config in ("sd3_fullft", "pixart_lora") and world > 1 and not args.tiny:
+        # every rank must time the SAME multiset of aspect buckets (ranks only start at different offsets in the bucket list),
+        # so the timed micro-batches must be whole cycles of it
+        nb, accum = (len(SD3_BUCKETS), 1) if args.config == "sd3_fullft" else (len(PIXART_BUCKETS), PIXART_GRAD_ACCUM)
+        cyc = nb // math.gcd(nb, accum)
+        if args.steps % cyc:
+            ap.error(f"--config {args.config} on {world} GPUs times whole bucket cycles: --steps must be a multiple of {cyc}")
+    sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree, not even bytecode of modules build() did not import
+    # torch seeds its global generators randomly per process; LoRA A init (kaiming_uniform_) and the VAE's sampling noise
+    # draw from them, so without this two runs with the same arguments would start from different inputs
+    torch.manual_seed(0)
     if args.dp == "auto" and args.config != "sd3_fullft":
         args.dp = "flat"
     if args.warmup < 3 and args.impl == "b200" and not args.tiny:
